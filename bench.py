@@ -15,11 +15,14 @@ proof).  One "step" = one pass of the hot path over one batch.  With N GPUs ever
             achieved = algorithmic bytes (N x (64-byte point + 32-byte scalar), SURVEY 8(d)) / kernel time vs the
             measured HBM copy peak.  The kernel is bound by the integer (IMAD) pipe, not HBM - see DESIGN.md.
   cpu_baseline: the CPU oracle port (oracle/zkref_*.c, all host threads) timed on ONE email of the same workload.
+  The inputs are seeded (RSA signing key, emails, proving key, blinding scalars r and s): the proofs repeat from run to
+  run, and `--dump-outputs DIR` writes those of the last timed step as .npy files for comparing two builds.
 
 `--impl reference` times that CPU path alone (the reference's snarkjs/circom stack is not runnable offline - DESIGN.md).
 """
 import argparse
 import ctypes
+import hashlib
 import json
 import os
 import subprocess
@@ -82,6 +85,23 @@ def make_inputs(z, circuit, count, key):
         dk = z.verify_dkim_signature(em, resolver=lambda n, t: [z.synthetic.key_record(key)])
         packed.append(circuit.pack_inputs(z.generate_email_verifier_inputs_from_dkim_result(dk)))
     return packed
+
+
+def dump_outputs(out_dir, proofs, publics, status, batch, npub):
+    """What one fullprove step returns, as .npy files: every 256-bit field element as its eight little-endian 32-bit
+    limbs in float64 (exact), so that the outputs of two builds can be compared element for element.
+      proofs.npy  [batch, 8, 8]     A.x, A.y, B.x.c0, B.x.c1, B.y.c0, B.y.c1, C.x, C.y of each proof
+      publics.npy [batch, npub, 8]  public signals
+      status.npy  [batch]           -1 = constraints satisfied, else the first violated constraint"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+
+    def limbs(raw, shape):
+        return np.frombuffer(raw, dtype="<u4").reshape(shape).astype(np.float64)
+
+    np.save(os.path.join(out_dir, "proofs.npy"), limbs(proofs, (batch, 8, 8)))
+    np.save(os.path.join(out_dir, "publics.npy"), limbs(publics, (batch, npub, 8)))
+    np.save(os.path.join(out_dir, "status.npy"), np.asarray(status, dtype=np.float64))
 
 
 def cpu_reference_proof(z, circuit, zk, packed_one, threads, rs=None):
@@ -237,7 +257,11 @@ def main():
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--skip-extra-configs", action="store_true",
                     help="do not measure BASELINE configs[3] / configs[4] / the sharded proof after the headline workload")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (proofs, public signals, status) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -262,7 +286,7 @@ def main():
     info = circuit.info
     N = 1 << info.domain_log2
     host_threads = os.cpu_count() or 1
-    key = z.synthetic.generate_key()
+    key = z.synthetic.generate_key(seed=KEY_SEED)
     zk = z.Zkey(circuit, seed=KEY_SEED, device=local_rank)
     config = {"workload": "configs[2]: batch of %d synthetic 1024-byte-body emails per GPU, EmailVerifier(1024,1536,121,17), "
                           "witness + full Groth16 prove" % args.batch,
@@ -305,14 +329,17 @@ def main():
     err = ctypes.create_string_buffer(4096)
     L = z._lib
     stream = torch.cuda.ExternalStream(ctx.stream, device=torch.device("cuda", local_rank))
+    # seeded blinding scalars (r, s) of every proof, in place of fresh randomness: the proofs repeat from run to run
+    blinding = b"".join((int.from_bytes(hashlib.sha256(b"bench %d %d" % (KEY_SEED, j)).digest(), "little") % z.FR_MODULUS).to_bytes(32, "little")
+                  for j in range(2 * batch))
 
     def step(inputs_ptr):
-        rc = L.zke_fullprove(ctx.handle, inputs_ptr, batch, None, pinned_proofs.data_ptr(), pinned_pub.data_ptr(), status, err, 4096)
+        rc = L.zke_fullprove(ctx.handle, inputs_ptr, batch, blinding, pinned_proofs.data_ptr(), pinned_pub.data_ptr(), status, err, 4096)
         if rc != 0:
             raise RuntimeError("zke_fullprove failed: %d %s" % (rc, err.value.decode()))
 
     def submit(inputs_ptr):
-        if L.zke_fullprove_submit(ctx.handle, inputs_ptr, batch, None, err, 4096) != 0:
+        if L.zke_fullprove_submit(ctx.handle, inputs_ptr, batch, blinding, err, 4096) != 0:
             raise RuntimeError("zke_fullprove_submit failed: %s" % err.value.decode())
 
     def collect():
@@ -363,12 +390,14 @@ def main():
     ms_e2e = timed(pinned_in.data_ptr(), args.steps)
     sampler.stop_flag = True
     sampler.join(timeout=2)
+    pr_raw, pb_raw = bytes(pinned_proofs.numpy()), bytes(pinned_pub.numpy())[: 32 * npub * batch]
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, pr_raw, pb_raw, list(status), batch, npub)
     # ---- every proof of the last end-to-end batch is verified (outside the timed region): the batch verifier checks them
     #      with one randomised product of pairings and falls back to one-by-one to name offenders
     proofs_verified = None
     if rank == 0:
         try:
-            pr_raw, pb_raw = bytes(pinned_proofs.numpy()), bytes(pinned_pub.numpy())
             t0 = time.perf_counter()
             items = [z.proof_to_json(pr_raw[256 * k: 256 * (k + 1)], pb_raw[32 * npub * k: 32 * npub * (k + 1)], npub) for k in range(batch)]
             oks = z.verify_batch(zk.vkey(), [it[1] for it in items], [it[0] for it in items])

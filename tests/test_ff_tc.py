@@ -7,6 +7,7 @@ The device routine itself is checked on the GPU against the integer product (scr
 through the bit-exact proof test test_tensor_core_reduction_h_msm_bit_exact."""
 import os
 import random
+import shutil
 import subprocess
 
 import pytest
@@ -47,7 +48,8 @@ def _expected_bfrag(p):
 @pytest.fixture(scope="module")
 def dump_binary(tmp_path_factory):
     exe = str(tmp_path_factory.mktemp("tc") / "tc_table_dump")
-    subprocess.check_call(["nvcc", "-O1", "-I", CSRC, "-o", exe, os.path.join(ROOT, "tests", "tc_table_dump.cu")])
+    nvcc = shutil.which("nvcc") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "nvcc")
+    subprocess.check_call([nvcc, "-O1", "-I", CSRC, "-o", exe, os.path.join(ROOT, "tests", "tc_table_dump.cu")])
     return exe
 
 

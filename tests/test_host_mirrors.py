@@ -121,6 +121,17 @@ def test_dkim_verify_roundtrip_and_failures():
         z.verify_dkim_signature(email)      # offline default resolver: no record from any source
 
 
+def test_seeded_key_repeats_and_signs():
+    """generate_key(seed=...) gives the same 2048-bit key on every call (benchmark inputs repeat from run to run)."""
+    key, again, other = (z.synthetic.generate_key(seed=s) for s in (7, 7, 8))
+    rec = z.synthetic.key_record(key)
+    assert rec == z.synthetic.key_record(again) and rec != z.synthetic.key_record(other)
+    assert key.key_size == 2048 and key.private_numbers().public_numbers.e == 65537
+    email = z.synthetic.make_signed_email(3, key)
+    assert email == z.synthetic.make_signed_email(3, again)
+    assert z.verify_dkim_signature(email, resolver=lambda n, t: [rec]).modulusLength == 2048
+
+
 def test_dkim_key_retry_and_sanitizers():
     """dkim/index.ts:49-66, :105-131 and dkim/sanitizers.ts: every key record of the selector is tried; when the first
     attempt ends in "bad signature" the sanitizers are tried in order and the passing one is reported."""

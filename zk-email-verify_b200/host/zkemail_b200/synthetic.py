@@ -4,6 +4,7 @@ generator", appendix A.10).  Headers follow the 7-field template of
 from __future__ import annotations
 import base64
 import hashlib
+import random
 
 import numpy as np
 from cryptography.hazmat.primitives import hashes, serialization
@@ -12,10 +13,48 @@ from cryptography.hazmat.primitives.asymmetric import padding, rsa
 from .dkim import format_relaxed_line, relaxed_body
 
 SEED_BASE = 0x5EED0000
+_SMALL_PRIMES = [p for p in range(3, 2000, 2) if all(p % q for q in range(3, int(p ** 0.5) + 1, 2))]
 
 
-def generate_key(bits: int = 2048):
-    return rsa.generate_private_key(public_exponent=65537, key_size=bits)
+def _probable_prime(n: int, rng: random.Random) -> bool:
+    if any(n % p == 0 for p in _SMALL_PRIMES):
+        return n in _SMALL_PRIMES
+    d, s = n - 1, 0
+    while d % 2 == 0:
+        d, s = d // 2, s + 1
+    for _ in range(40):                                  # Miller-Rabin
+        x = pow(rng.randrange(2, n - 1), d, n)
+        if x in (1, n - 1):
+            continue
+        for _ in range(s - 1):
+            x = pow(x, 2, n)
+            if x == n - 1:
+                break
+        else:
+            return False
+    return True
+
+
+def generate_key(bits: int = 2048, seed: int | None = None):
+    """A fresh RSA key, or with `seed` the same key on every call, so that benchmark inputs repeat from run to run."""
+    e = 65537
+    if seed is None:
+        return rsa.generate_private_key(public_exponent=e, key_size=bits)
+    rng = random.Random(seed)
+
+    def prime():
+        while True:
+            c = rng.getrandbits(bits // 2) | (3 << (bits // 2 - 2)) | 1     # top two bits set: n has exactly `bits` bits
+            if c % e != 1 and _probable_prime(c, rng):
+                return c
+
+    p = prime()
+    q = prime()
+    while q == p:
+        q = prime()
+    d = pow(e, -1, (p - 1) * (q - 1))
+    return rsa.RSAPrivateNumbers(p, q, d, rsa.rsa_crt_dmp1(d, p), rsa.rsa_crt_dmq1(d, q), rsa.rsa_crt_iqmp(p, q),
+                                 rsa.RSAPublicNumbers(e, p * q)).private_key()
 
 
 def key_record(key) -> str:
